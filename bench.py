@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - synthesized audio samples/sec @ batch 64 + VQ-index bit-exact rate (BASELINE.json metric, config C4).
 
-    python bench.py --gpus N --steps K --warmup W [--impl b200|reference|torch_gpu] [--config c4|c2]
+    python bench.py --gpus N --steps K --warmup W [--impl b200|reference|torch_gpu] [--config c4|c2|c3] [--dump-outputs DIR]
 
 One "step" = one pass of the synthesis hot path over one batch of 64 synthetic utterances U
 (SURVEY.md §8: 64 phones, 8-s prompt -> 500 mel frames, durations forced to 8 -> 512 mel
@@ -26,6 +26,11 @@ Arms:  --impl b200       the product (this repo's CUDA path)                    
 
 Output: ONE JSON line (contract in the task statement) with `roofline`, `cpu_baseline`, `e2e`, `clocks`,
 `gpu_launches` and the parity half of the metric: `vq_index_bit_exact_rate`, `duration_exact_rate`, `mel_l1`.
+
+--dump-outputs DIR (product arm): after the timed steps, what the last timed step returned to its caller is written as
+DIR/<name>.npy - c4: `wav` (batch, 1, samples) of rank 0's shard; c2: `mel` (clips, 80, frames); c3: `ids` (16, 512) -
+in float32 (ids in float64, exact).  Inputs and weights are seeded, so two builds run with the same arguments can be
+compared array for array.  An output larger than DUMP_BYTES is cut to a fixed, seeded sample of its rows (dim 0).
 """
 import argparse
 import ctypes as C
@@ -69,11 +74,40 @@ def parse():
     ap.add_argument("--cpu-workers", type=int, default=0, help="concurrent batch-1 CPU workers (0 = cpus / 16, at most 4)")
     ap.add_argument("--cpu-threads", type=int, default=0, help="torch threads per CPU worker (0 = 16)")
     ap.add_argument("--clips", type=int, default=10000, help="--config c2: number of 3-s clips")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the product's outputs (--impl b200)")
+    return args
 
 
 def log(*a):
     print("[bench]", *a, file=sys.stderr, flush=True)
+
+
+DUMP_BYTES = 64 * 10**6                               # --dump-outputs: at most this many bytes over all arrays
+DUMP_SEED = 0
+
+
+def dump_outputs(d, arrays):
+    """arrays {name: tensor} -> d/<name>.npy: floating point as float32, integers as float64 (exact).  An array over its
+    share of DUMP_BYTES keeps a sample of its rows (dim 0), in order, drawn from DUMP_SEED: the same rows on every run."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        t = t.float() if t.is_floating_point() else t.double()
+        row_bytes = t[0].numel() * t.element_size()
+        if t.numel() * t.element_size() > share:
+            keep = share // row_bytes
+            rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(DUMP_SEED))[:keep].sort().values
+            log(f"dump: {name} keeps a seeded sample of {keep} of its {t.shape[0]} rows")
+            t = t[rows]
+        np.save(os.path.join(d, name + ".npy"), t.numpy())
+        log(f"dump: {os.path.join(d, name + '.npy')} {tuple(t.shape)} {t.dtype}")
 
 
 def peaks():
@@ -297,6 +331,7 @@ def run_b200(args):
         out = gpu_step(tts, wav_d, phone_d, forced_d, revocode)
     e1.record()
     barrier()
+    timed_out = out if args.dump_outputs else None
     clocks = sampler.stop() if rank == 0 else None
     launches = ops.launch_count() - n0
     ms = e0.elapsed_time(e1)
@@ -316,6 +351,8 @@ def run_b200(args):
     barrier()
     ms_e2e = f0.elapsed_time(f1)
     log(f"e2e region: {ms_e2e / args.steps:.1f} ms/step")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"wav": timed_out})
 
     if dist is not None:
         t = torch.tensor([ms, ms_e2e], device=dev)
@@ -614,6 +651,8 @@ def run_c2(args):
     f1.record()
     torch.cuda.synchronize()
     ms_e2e = f0.elapsed_time(f1) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"mel": mel})
     pk, pk_src = peaks()
     bytes_per_clip = Ls * 4 + 80 * (1 + Ls // 256) * 4
     gbs = n * bytes_per_clip / (ms / 1e3) / 1e9
@@ -662,7 +701,7 @@ def run_c3(args):
     for _ in range(max(1, min(args.warmup, 2))):
         ids = tts.plm.infer(tc)
     torch.cuda.synchronize()
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     n0 = ops.launch_count()
     sampler = ClockSampler(0)
     sampler.start()
@@ -683,6 +722,8 @@ def run_c3(args):
     f1.record()
     torch.cuda.synchronize()
     ms_e2e = f0.elapsed_time(f1) / steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"ids": ids})
     # roofline leg: algorithmic FLOPs and CUDA-event time of the tap-GEMM launches of ONE decode (eager enqueue)
     lib = L.lib()
     lib.mtts_profile_begin()

@@ -136,14 +136,15 @@ def test_hifigan_shape_and_regression(golden, weights_cpu):
     assert n == 13_926_017                 # HiFi-GAN V1 generator size (SURVEY.md §8c)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/modules"), reason="reference tree not present (GPU box)")
-def test_reference_loads_oracle_weights_strict():
-    """Container only: the real reference accepts the oracle's state dicts with strict=True."""
-    from oracle import stubs
-    G, plm, adm = stubs.build_reference_models()
-    G.load_state_dict(weights.g_state_dict(), strict=True)
-    plm.load_state_dict(weights.plm_state_dict(), strict=True)
-    adm.load_state_dict(weights.adm_state_dict(), strict=True)
+def test_reference_loads_oracle_weights_strict(weights_cpu):
+    """The real reference accepts the oracle's state dicts with strict=True: the same keys, each with the shape of the
+    reference's own tensor.  The reference's layout is the one oracle/make_golden.py recorded from its modules."""
+    with open(os.path.join(GOLDEN, "state_dict_keys.json")) as f:
+        ref = json.load(f)
+    for name, sd in (("G", weights_cpu("g")), ("plm", weights_cpu("plm")), ("adm", weights_cpu("adm"))):
+        assert sorted(sd) == sorted(ref[name]), name
+        assert {k: list(v.shape) for k, v in sd.items()} == ref[name], name
+        assert all(v.dtype == torch.float32 for v in sd.values()), name
 
 
 def test_c_oracle_vq_matches_reference_fixture(golden, weights_cpu):

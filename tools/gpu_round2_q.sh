@@ -2,6 +2,7 @@
 # GPU call Q: MMA cost with uniform issue (cta_group::1 / ::2), two-heads-per-CTA tensor-core attention: parity + A/B
 set -u
 mkdir -p gpurun_out
+nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o tools/microbench/mma_floor2 tools/microbench/mma_floor2.cu
 ./tools/microbench/mma_floor2 2>&1 | tee gpurun_out/r2q_mma_floor2.log
 timeout 600 python -m pytest tests/test_gpu_parity.py -q -m gpu -k "attention" --timeout 300 -p no:randomly 2>&1 | tail -5
 for pm in 1000 16; do
