@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define MTTS_ABI_VERSION 3
+#define MTTS_ABI_VERSION 4
 
 typedef enum {
   MTTS_OK = 0,
@@ -60,16 +60,6 @@ int mtts_trace_end(char* buf, int32_t buf_len);
  * and reruns the batch on BF16X3. */
 enum { MTTS_TC_BF16X3 = 0, MTTS_TC_F16X2 = 1 };
 int mtts_tc_overflow_bind(int32_t* flag_dev);
-/* SM budget of the calling host thread's subsequent launches (0 = the whole device): the persistent tensor-core kernels
- * size their grids from it, so work enqueued on two streams can share the device (the prompt re-vocode of Megatts.forward
- * runs beside the latency-bound AR loops). */
-int mtts_set_sm_limit(int32_t n_sms);
-/* Launch policy of the calling host thread while two streams share the device: SM budget (as above), whether the dense
- * layers may run as CTA pairs (cta_group::2 clusters need two free SMs of one TPC), and whether launches carry the
- * programmatic-dependent-launch attribute (a long kernel's successor would otherwise be scheduled early onto the SMs left
- * free for the other stream).  (0, 1, 1) restores the defaults.  Megatts.synthesize uses it to re-vocode the prompt
- * (models/megatts2.py:371-372 of the reference) beside the MRTE + ADM stages. */
-int mtts_set_launch_policy(int32_t sm_limit, int32_t allow_pairs, int32_t allow_pdl);
 /* Diagnostics (host only, no CUDA call): the launch plan the tap-GEMM dispatcher picks for a stride-1 layer of this shape
  * (B x T output rows, k taps) on n_sms SMs, with partial_bytes of split-K partial-sum space and, if ln_rides, a LayerNorm
  * that the split's reduction can carry.  out5 = {N-tile width, K splits, CTA pair, halo form (0 | 1 | 2 = as a pair),
@@ -175,10 +165,6 @@ typedef struct {
   int32_t o_planes_fmt;                    /* MTTS_TC_BF16X3 | MTTS_TC_F16X2 */
 } mtts_attn_params;
 int mtts_attention_f32(const mtts_attn_params* p, void* stream);
-/* Opt-in: AR-step attention (Tq == Tk <= 64, even head count, dh 64 | 96) with at least `min_len` rows runs on the
- * two-heads-per-CTA tcgen05 kernel instead of the fp32 kernel; min_len <= 0 switches it off (the default: it is slower
- * inside the synthesis step, see csrc/ops.cu).  Returns the previous setting. */
-int mtts_set_attention_pair_min(int32_t min_len);
 
 /* EuclideanCodebook.quantize (modules/quantization/core_vq.py:175-183): first index of
  * max_k -(|x|^2 - 2 x.e_k + |e_k|^2).  x (N, D) ld = ldx, embed (K, D) -> idx (N) int64 */

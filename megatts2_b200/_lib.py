@@ -9,7 +9,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libmegatts2_b200.so")
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 ACT_NONE, ACT_RELU, ACT_LEAKY, ACT_TANH = 0, 1, 2, 3
 TC_BF16X3, TC_F16X2 = 0, 1
 PAD_ZERO, PAD_REFLECT, PAD_REPLICATE = 0, 1, 2
@@ -118,10 +118,7 @@ SIGNATURES = {
     "mtts_linear_tc_f32": (C.c_int, [vp, i32, i64, i32, vp, i32, vp, vp, i32, vp, i32, i32, f32, i32, vp, i64, i64, i32, vp]),
     "mtts_split_planes_f32": (C.c_int, [vp, i32, i64, i32, vp, i32, vp]),
     "mtts_tc_overflow_bind": (C.c_int, [vp]),
-    "mtts_set_sm_limit": (C.c_int, [i32]),
-    "mtts_set_launch_policy": (C.c_int, [i32, i32, i32]),
     "mtts_tc_plan_query": (C.c_int, [i32, i32, i32, i32, i32, i32, i32, i32, i64, i32, C.POINTER(i32)]),
-    "mtts_set_attention_pair_min": (C.c_int, [i32]),
     "mtts_mask_tail_f32": (C.c_int, [vp, i32, i32, i32, vp, vp]),
     "mtts_resample_f32": (C.c_int, [vp, i64, i32, i32, vp, vp, i32, i32, i32, i32, vp, i64, i32, vp, vp]),
     "mtts_peak_normalize_f32": (C.c_int, [vp, i64, i32, i32, vp, vp, vp]),

@@ -15,14 +15,12 @@ namespace mtts {
 thread_local char g_err[512] = "";
 std::atomic<int64_t> g_launches{0};
 
-static thread_local bool g_thread_pdl = true;     // per host thread: set_launch_policy() (conv_tc.cu)
-void set_thread_pdl(bool on) { g_thread_pdl = on; }
 bool pdl_enabled() {
   static const bool on = [] {
     const char* e = getenv("MEGATTS2_PDL");
     return !(e && e[0] == '0');
   }();
-  return on && g_thread_pdl;
+  return on;
 }
 
 bool g_trace_on = false;

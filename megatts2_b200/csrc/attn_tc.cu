@@ -313,245 +313,6 @@ int attn_tc_launch(const mtts_attn_params& p, cudaStream_t st) {
   return 0;
 }
 
-// ------------------------------------------------------------------------------------------------------------------
-// Short sequences (the AR steps: Tq == Tk <= 64): TWO heads per CTA.  A head alone is a 64 x 64 x dh problem and fills half
-// of a 128-row MMA; here thread r owns query row (r & 63) of head 2 * blockIdx.x + (r >> 6).  The two heads are stacked:
-//   S = [Q_a; Q_b] [K_a; K_b]^T   one 128 x 128 x dh product whose off-diagonal 64 x 64 blocks (head a against head b) are
-//                                 simply never read,
-//   O = [P_a 0; 0 P_b] [V_a; V_b] one 128 x dh x 128 product with the block-diagonal P written by the softmax threads.
-// A single key tile, so no online-softmax rescale.  P reuses the Q | K staging area (both are dead once S has been
-// computed); with dh = 64 the CTA needs 97 KB and 256 TMEM columns, so two CTAs share an SM and one's staging / softmax
-// overlaps the other's MMAs.
-template <int DH>
-struct AtpCfg {
-  static constexpr int NS = DH / 32;                      // 64-byte K-slabs along dh
-  static constexpr int R_SLAB = 128 * 64;                 // 128 rows x 64 B (Q, K and P slabs)
-  static constexpr int V_SLAB = DH * 64;                  // V^T: dh rows, one slab per 32 keys, 4 slabs (128 stacked keys)
-  static constexpr int Q_PLANE = NS * R_SLAB, V_PLANE = 4 * V_SLAB, P_PLANE = 4 * R_SLAB;
-  static constexpr int OFF_Q = 0, OFF_K = 2 * Q_PLANE;
-  static constexpr int QK_BYTES = 4 * Q_PLANE, P_BYTES = 2 * P_PLANE;
-  static constexpr int OFF_P = 0;                         // aliases Q | K
-  static constexpr int OFF_V = QK_BYTES > P_BYTES ? QK_BYTES : P_BYTES;
-  static constexpr int OFF_BAR = OFF_V + 2 * V_PLANE;
-  static constexpr int SMEM = OFF_BAR + 1024 + 64;        // + alignment slack + barrier / TMEM slot
-  static constexpr int TMEM_COLS = 256;                   // S: 128 main + 128 correction; O (2 * dh <= 256) reuses them
-};
-
-template <int DH>
-__global__ void __launch_bounds__(128)
-attn_tc_pair_kernel(const mtts_attn_params p, int32_t* ovf) {
-  using Cfg = AtpCfg<DH>;
-  pdl_trigger();
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* sm = smem_raw + (base - smem_u32(smem_raw));
-  const uint32_t bar = base + Cfg::OFF_BAR;
-  const uint32_t tmem_slot = bar + 16;
-  uint32_t* tmem_slot_ptr = reinterpret_cast<uint32_t*>(sm + Cfg::OFF_BAR + 16);
-
-  const int tid = threadIdx.x;
-  const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
-  const int hh = tid >> 6, row = tid & 63;
-  const int h = 2 * blockIdx.x + hh, b = blockIdx.y;
-  const int S = p.Tk;                                      // == Tq <= 64
-  const bool valid = row < S;
-
-  if (tid == 0) {
-    mbar_init(bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "n"(Cfg::TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  pdl_wait();
-  bool bad = false;
-  // ---- stage Q and K: thread r splits row r of each stacked operand (rows past S are zero)
-  {
-    const float* qsrc = p.q + (int64_t)b * p.q_sb + (int64_t)(valid ? row : 0) * p.q_st + (int64_t)h * DH;
-    const float* ksrc = p.k + (int64_t)b * p.k_sb + (int64_t)(valid ? row : 0) * p.k_st + (int64_t)h * DH;
-#pragma unroll
-    for (int c8 = 0; c8 < DH / 8; ++c8) {
-      float vq[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, vk[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-      if (valid) {
-        const float4 a = *reinterpret_cast<const float4*>(qsrc + c8 * 8), c = *reinterpret_cast<const float4*>(qsrc + c8 * 8 + 4);
-        const float4 d = *reinterpret_cast<const float4*>(ksrc + c8 * 8), e = *reinterpret_cast<const float4*>(ksrc + c8 * 8 + 4);
-        vq[0] = a.x; vq[1] = a.y; vq[2] = a.z; vq[3] = a.w; vq[4] = c.x; vq[5] = c.y; vq[6] = c.z; vq[7] = c.w;
-        vk[0] = d.x; vk[1] = d.y; vk[2] = d.z; vk[3] = d.w; vk[4] = e.x; vk[5] = e.y; vk[6] = e.z; vk[7] = e.w;
-      }
-      uint4 p0, p1;
-      const uint32_t off = (uint32_t)(c8 >> 2) * Cfg::R_SLAB + sw64_off(tid, c8 & 3);
-      split8_f16x2(vq, p0, p1, bad);
-      *reinterpret_cast<uint4*>(sm + Cfg::OFF_Q + off) = p0;
-      *reinterpret_cast<uint4*>(sm + Cfg::OFF_Q + Cfg::Q_PLANE + off) = p1;
-      split8_f16x2(vk, p0, p1, bad);
-      *reinterpret_cast<uint4*>(sm + Cfg::OFF_K + off) = p0;
-      *reinterpret_cast<uint4*>(sm + Cfg::OFF_K + Cfg::Q_PLANE + off) = p1;
-    }
-  }
-  // ---- stage V^T: thread r transposes key (r & 63) of its head into column r of the (dh x 128) operand; a warp's 32
-  //      lanes fill one 64-byte row with 2-byte stores
-  {
-    const float* src = p.v + (int64_t)b * p.v_sb + (int64_t)(valid ? row : 0) * p.v_st + (int64_t)h * DH;
-    uint8_t* vt0 = sm + Cfg::OFF_V + (tid >> 5) * Cfg::V_SLAB;
-    const int kk = tid & 31;
-#pragma unroll
-    for (int i = 0; i < DH / 4; ++i) {
-      float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (valid) a = *reinterpret_cast<const float4*>(src + i * 4);
-      const float vv[4] = {a.x, a.y, a.z, a.w};
-#pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        const int d = i * 4 + e;
-        const __half x1 = __float2half_rn(vv[e]);
-        const __half x2 = __float2half_rn((vv[e] - __half2float(x1)) * F16X2_SCALE);
-        bad |= !(fabsf(vv[e]) <= 65504.0f);
-        const uint32_t off = sw64_off(d, kk >> 3) + (uint32_t)(kk & 7) * 2u;
-        *reinterpret_cast<uint16_t*>(vt0 + off) = __half_as_ushort(x1);
-        *reinterpret_cast<uint16_t*>(vt0 + Cfg::V_PLANE + off) = __half_as_ushort(x2);
-      }
-    }
-  }
-  fence_proxy_async_smem();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = __shfl_sync(0xffffffffu, *tmem_slot_ptr, 0);
-  const uint32_t leader = (warp == 0 && elect_one()) ? 1u : 0u;
-  const uint32_t lane_addr = tmem + ((uint32_t)(warp * 32) << 16);
-  const uint64_t desc_hi = umma_desc_kmajor<64>(0u);
-  constexpr uint32_t IDESC_S = (1u << 4) | ((uint32_t)(128 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);   // f16 x f16 -> f32, N 128
-  constexpr uint32_t IDESC_O = (1u << 4) | ((uint32_t)(DH >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);    // N dh
-
-  // ---- S = [Q_a; Q_b] [K_a; K_b]^T
-  if (warp == 0) {
-#pragma unroll
-    for (int ks = 0; ks < DH / 16; ++ks) {
-      const uint32_t qa = base + Cfg::OFF_Q + (ks >> 1) * Cfg::R_SLAB + (ks & 1) * 32;
-      const uint32_t ka = base + Cfg::OFF_K + (ks >> 1) * Cfg::R_SLAB + (ks & 1) * 32;
-      const uint64_t a1 = desc_hi | (uint64_t)((qa >> 4) & 0x3FFF), a2 = desc_hi | (uint64_t)(((qa + Cfg::Q_PLANE) >> 4) & 0x3FFF);
-      const uint64_t b1 = desc_hi | (uint64_t)((ka >> 4) & 0x3FFF), b2 = desc_hi | (uint64_t)(((ka + Cfg::Q_PLANE) >> 4) & 0x3FFF);
-      tc_mma_l(tmem + 128, a1, b2, IDESC_S, ks ? 1u : 0u, leader);      // correction: q1 k2' + q2' k1
-      tc_mma_l(tmem + 128, a2, b1, IDESC_S, 1u, leader);
-      tc_mma_l(tmem, a1, b1, IDESC_S, ks ? 1u : 0u, leader);            // main: q1 k1
-    }
-    tc_commit_l(bar, leader);
-  }
-  mbar_wait(bar, 0);
-  tc_fence_after();
-  // ---- softmax over this thread's row: its own head's 64 columns
-  const float* mrow = p.mask ? p.mask + (int64_t)b * p.mask_sb + (int64_t)h * p.mask_sh + (int64_t)(valid ? row : 0) * p.mask_sq : nullptr;
-  float s[64];
-#pragma unroll
-  for (int u = 0; u < 4; ++u) {
-    uint32_t r[16], rc[16];
-    tmem_ld16(lane_addr + hh * 64 + u * 16, r);
-    tmem_ld16(lane_addr + 128 + hh * 64 + u * 16, rc);
-    tmem_ld_wait();
-#pragma unroll
-    for (int j = 0; j < 16; ++j) {
-      const int key = u * 16 + j;
-      float x = fmaf(__uint_as_float(rc[j]), F16X2_INV_SCALE, __uint_as_float(r[j])) * p.scale;
-      if (mrow && key < S) x += mrow[key];
-      s[key] = key < S ? x : -INFINITY;
-    }
-  }
-  float m = s[0];
-#pragma unroll
-  for (int j = 1; j < 64; ++j) m = fmaxf(m, s[j]);
-  const float m_use = (m == -INFINITY) ? 0.f : m;
-  float l = 0.f;
-#pragma unroll
-  for (int j = 0; j < 64; ++j) {
-    s[j] = expf(s[j] - m_use);
-    l += s[j];
-  }
-  // P row r: columns [64 hh, 64 hh + 64) hold this head's probabilities, the other head's 64 columns are zero
-  {
-    bool pbad = false;     // p is in [0, 1]: never out of range
-    const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
-#pragma unroll
-    for (int c8 = 0; c8 < 8; ++c8) {
-      uint4 p0, p1;
-      split8_f16x2(s + c8 * 8, p0, p1, pbad);
-      const int cm = hh * 8 + c8, cz = (1 - hh) * 8 + c8;       // 16-byte chunk index along the 128 stacked keys
-      const uint32_t off = (uint32_t)(cm >> 2) * Cfg::R_SLAB + sw64_off(tid, cm & 3);
-      const uint32_t offz = (uint32_t)(cz >> 2) * Cfg::R_SLAB + sw64_off(tid, cz & 3);
-      *reinterpret_cast<uint4*>(sm + Cfg::OFF_P + off) = p0;
-      *reinterpret_cast<uint4*>(sm + Cfg::OFF_P + Cfg::P_PLANE + off) = p1;
-      *reinterpret_cast<uint4*>(sm + Cfg::OFF_P + offz) = zero;
-      *reinterpret_cast<uint4*>(sm + Cfg::OFF_P + Cfg::P_PLANE + offz) = zero;
-    }
-  }
-  fence_proxy_async_smem();
-  tc_fence_before();       // this thread's reads of S are complete before O overwrites the columns
-  __syncthreads();
-  // ---- O = P [V_a; V_b]   (K = 128 stacked keys: 8 k-steps)
-  if (warp == 0) {
-    tc_fence_after();
-#pragma unroll
-    for (int ks = 0; ks < 8; ++ks) {
-      const uint32_t pa = base + Cfg::OFF_P + (ks >> 1) * Cfg::R_SLAB + (ks & 1) * 32;
-      const uint32_t va = base + Cfg::OFF_V + (ks >> 1) * Cfg::V_SLAB + (ks & 1) * 32;
-      const uint64_t a1 = desc_hi | (uint64_t)((pa >> 4) & 0x3FFF), a2 = desc_hi | (uint64_t)(((pa + Cfg::P_PLANE) >> 4) & 0x3FFF);
-      const uint64_t b1 = desc_hi | (uint64_t)((va >> 4) & 0x3FFF), b2 = desc_hi | (uint64_t)(((va + Cfg::V_PLANE) >> 4) & 0x3FFF);
-      tc_mma_l(tmem + DH, a1, b2, IDESC_O, ks ? 1u : 0u, leader);
-      tc_mma_l(tmem + DH, a2, b1, IDESC_O, 1u, leader);
-      tc_mma_l(tmem, a1, b1, IDESC_O, ks ? 1u : 0u, leader);
-    }
-    tc_commit_l(bar, leader);
-  }
-  mbar_wait(bar, 1);
-  tc_fence_after();
-  if (bad && ovf) *ovf = 1;
-  // ---- output: this thread's row, 16 columns at a time
-  {
-    const float inv = 1.0f / l;
-    float* o = p.o ? p.o + (int64_t)b * p.o_sb + (int64_t)row * p.o_st + (int64_t)h * DH : nullptr;
-    __nv_bfloat16* pl = reinterpret_cast<__nv_bfloat16*>(p.o_planes);
-    const int64_t poff = ((int64_t)b * p.Tq + row) * p.o_planes_ld + (int64_t)h * DH;
-#pragma unroll
-    for (int u = 0; u < DH / 16; ++u) {
-      uint32_t r[16], rc[16];
-      tmem_ld16(lane_addr + u * 16, r);
-      tmem_ld16(lane_addr + DH + u * 16, rc);
-      tmem_ld_wait();
-      if (valid) {
-#pragma unroll
-        for (int j = 0; j < 16; j += 4) {
-          float v[4];
-#pragma unroll
-          for (int e = 0; e < 4; ++e) v[e] = fmaf(__uint_as_float(rc[j + e]), F16X2_INV_SCALE, __uint_as_float(r[j + e])) * inv;
-          if (o) *reinterpret_cast<float4*>(o + u * 16 + j) = make_float4(v[0], v[1], v[2], v[3]);
-          if (pl) store_planes4(pl, p.o_plane_stride, poff + u * 16 + j, v, p.o_planes_fmt, ovf);
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(Cfg::TMEM_COLS) : "memory");
-  }
-}
-
-template <int DH>
-int attn_tc_pair_launch(const mtts_attn_params& p, cudaStream_t st) {
-  using Cfg = AtpCfg<DH>;
-  static std::atomic<uint64_t> configured{0};
-  const int dev = cur_device();
-  if (!(configured.load(std::memory_order_relaxed) & (1ull << dev))) {
-    cudaError_t e = cudaFuncSetAttribute(attn_tc_pair_kernel<DH>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM);
-    if (e != cudaSuccess) return fail(MTTS_ERR_CUDA, "%s: cudaFuncSetAttribute failed: %lld", "attention_tc_pair", (long long)e);
-    configured.fetch_or(1ull << dev, std::memory_order_relaxed);
-  }
-  dim3 grid((unsigned)(p.H / 2), (unsigned)p.B);
-  launch_k(attn_tc_pair_kernel<DH>, grid, 128, Cfg::SMEM, st, p, tc_ovf_ptr());
-  MTTS_CHECK_LAUNCH();
-  return 0;
-}
-
 }  // namespace
 
 // eligible: head dims of the AR stacks, 16-byte aligned fp32 views, output rows aligned for float4 / plane stores
@@ -564,16 +325,6 @@ bool attention_tc_eligible(const mtts_attn_params& p) {
   if (p.o && !(al(p.o) && p.o_st % 4 == 0 && p.o_sb % 4 == 0)) return false;
   if (p.o_planes && (p.o_planes_ld % 4 != 0 || p.o_plane_stride % 4 != 0)) return false;
   return p.B > 0 && p.H > 0 && p.Tq > 0 && p.Tk > 0 && p.H <= 65535 && p.B <= 65535;
-}
-
-// the two-heads-per-CTA form: an AR step (every query sees every key of an equally long sequence of at most 64 rows)
-bool attention_tc_pair_eligible(const mtts_attn_params& p) {
-  return (p.dh == 64 || p.dh == 96) && p.Tq == p.Tk && p.Tk <= 64 && (p.H % 2) == 0 && attention_tc_eligible(p);
-}
-
-int attention_tc_pair(const mtts_attn_params& p, cudaStream_t st) {
-  MTTS_REQUIRE(attention_tc_pair_eligible(p), "shape / alignment not eligible for the two-head tensor-core attention");
-  return p.dh == 64 ? attn_tc_pair_launch<64>(p, st) : attn_tc_pair_launch<96>(p, st);
 }
 
 int attention_tc(const mtts_attn_params& p, cudaStream_t st) {

@@ -56,7 +56,6 @@ __device__ __forceinline__ void pdl_entry() {
   pdl_wait();
 }
 bool pdl_enabled();
-void set_thread_pdl(bool on);
 template <typename... KArgs, typename... Args>
 inline void launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg = {};

@@ -20,8 +20,6 @@
 #include <mutex>
 #include <unordered_map>
 
-#include <stdlib.h>
-
 #include "kernels.h"
 #include "tc_ptx.cuh"
 
@@ -45,7 +43,6 @@ struct ConvTcArgs {
   int32_t splits; float* partial;
   int32_t fmt; int32_t* ovf;   // operand format of the plane output (== the kernel's own NP) and the f16 range flag
   int32_t row0;                // first padded row of this conv inside a shared plane buffer (0 for its own planes)
-  int32_t bo_mode;             // halo form, diagnostics: 1 = put (addr >> 7) & 7 into the descriptors' base-offset field (WRONG on B200)
 };
 
 // PAIR = 1: two CTAs of a cluster run one 256 x BN tile with cta_group::2 MMAs; each CTA stages its own 128 rows of
@@ -299,7 +296,7 @@ conv_tc_kernel(const __grid_constant__ ConvTcMaps maps, const ConvTcArgs g) {
 #pragma unroll
             for (int ks = 0; ks < Cfg::BK / 16; ++ks) {
               const uint32_t aa = a_addr + ks * 32, bb = b_addr + ks * 32;
-              const uint64_t a1 = umma_desc_shifted(desc_base, aa, g.bo_mode), a2 = umma_desc_shifted(desc_base, aa + Cfg::A_PLANE, g.bo_mode);
+              const uint64_t a1 = umma_desc_shifted(desc_base, aa), a2 = umma_desc_shifted(desc_base, aa + Cfg::A_PLANE);
               const uint64_t b1 = desc_base | (uint64_t)((bb >> 4) & 0x3FFF), b2 = desc_base | (uint64_t)(((bb + Cfg::B_PLANE) >> 4) & 0x3FFF);
               const uint32_t f = (ks == 0) ? first : 1u;
               if constexpr (NP == 2) {
@@ -313,7 +310,7 @@ conv_tc_kernel(const __grid_constant__ ConvTcMaps maps, const ConvTcArgs g) {
                   tc_mma_l(d_main, a1, b1, idesc, f, leader);
                 }
               } else {
-                const uint64_t a3 = umma_desc_shifted(desc_base, aa + 2 * Cfg::A_PLANE, g.bo_mode);
+                const uint64_t a3 = umma_desc_shifted(desc_base, aa + 2 * Cfg::A_PLANE);
                 const uint64_t b3 = desc_base | (uint64_t)(((bb + 2 * Cfg::B_PLANE) >> 4) & 0x3FFF);
                 if constexpr (PAIR) {
                   tc_mma_2sm_l(d_corr, a2, b2, idesc, f, leader);
@@ -757,29 +754,6 @@ int cur_device() {
   cudaGetDevice(&dev);
   return dev < 0 || dev >= MAX_DEV ? 0 : dev;
 }
-// SM budget of the calling host thread's launches (0 = the whole device).  The persistent tensor-core kernels size their
-// grids from it, so two streams can share the device: the vocoder pass that re-vocodes the prompt runs on a side stream
-// with a reduced budget while the latency-bound AR loops use the SMs it leaves free (models/megatts2.py).
-static thread_local int g_sm_limit = 0;
-static thread_local bool g_pairs_off = false;
-int set_sm_limit(int n) {
-  g_sm_limit = n > 0 ? n : 0;
-  return 0;
-}
-// Launch policy of the calling host thread while two streams share the device (models/megatts2.py, the prompt re-vocode beside
-// the MRTE + ADM stages).  Three rules make the sharing work; without any one of them the short launches of one stream queue
-// behind ~1 ms persistent CTAs of the other (the budget-only form measured 447 ... 660 ms against 421 ms sequential,
-// profiles/r2j_revocode_overlap_sweep.log):
-//  * the budgets of the two streams add up to the device (a persistent grid sized for all SMs waits for the other stream's CTAs);
-//  * no programmatic dependent launch on the stream with the long kernels: its NEXT kernel's CTAs would be scheduled early onto
-//    the SMs left free for the other stream and sit there in griddepcontrol.wait until the current kernel has finished;
-//  * no CTA pairs on the stream with the short kernels: the long stream's single CTAs leave free SMs, not free SM pairs.
-int set_launch_policy(int sm_limit, int allow_pairs, int allow_pdl) {
-  g_sm_limit = sm_limit > 0 ? sm_limit : 0;
-  g_pairs_off = allow_pairs == 0;
-  set_thread_pdl(allow_pdl != 0);
-  return 0;
-}
 int cur_device_sms() {
   const int dev = cur_device();
   if (!g_dev[dev].sms) {
@@ -787,50 +761,12 @@ int cur_device_sms() {
     cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
     g_dev[dev].sms = n > 0 ? n : 1;
   }
-  const int all = g_dev[dev].sms;
-  return g_sm_limit > 0 && g_sm_limit < all ? g_sm_limit : all;
+  return g_dev[dev].sms;
 }
 int32_t* tc_ovf_ptr() { return g_dev[cur_device()].ovf; }
 int tc_overflow_bind(int32_t* flag) {
   g_dev[cur_device()].ovf = flag;
   return 0;
-}
-
-// tuning switches (diagnostics), read ONCE per process: MEGATTS2_TC_SPLITK = 0 disables split-K, _SPLITK_MAX / _SPLITK_MARGIN
-// tune its cost model, MEGATTS2_TC_PAIR = 0 | 1 | 2 | 3 | 4 (0: no CTA pairs, 2 / 4: 32-wide K-slabs, 3 / 4: pairs for convs
-// too), MEGATTS2_TC_SWB64 = 1 forces 64-byte swizzle rows
-struct CtcEnv { bool splitk; int sk_max; double margin; double ln_red; int pair_mode; bool swb64; bool halo; int halo_bo; int halo_pair; int model; };
-static const CtcEnv& ctc_env() {
-  static const CtcEnv env = [] {
-    CtcEnv e;
-    const char* ke = getenv("MEGATTS2_TC_SPLITK");
-    const char* me = getenv("MEGATTS2_TC_SPLITK_MAX");
-    const char* ge = getenv("MEGATTS2_TC_SPLITK_MARGIN");
-    const char* pe = getenv("MEGATTS2_TC_PAIR");
-    const char* se = getenv("MEGATTS2_TC_SWB64");
-    e.splitk = !(ke && ke[0] == '0');
-    e.sk_max = me ? atoi(me) : 8;
-    e.margin = ge ? atof(ge) : 0.85;
-    // modelled cycles of a reduction that REPLACES the LayerNorm launch that would follow anyway (tc_splitk_reduce_ln_kernel):
-    // 2000 instead of the plain reduction's 9000 makes the out-projection / FF2 layers split up to steps 18 (PLM) / 24 (ADM):
-    // every affected step got faster, PLM -0.4 ms, ADM -1.0 ms per decode (gpurun call LN, profiles/r3d_lncost_curves.log)
-    const char* le = getenv("MEGATTS2_TC_SPLITK_LNCOST");
-    e.ln_red = le ? atof(le) : 2000.0;
-    e.pair_mode = pe ? atoi(pe) : 1;
-    e.swb64 = se && se[0] == '1';
-    const char* he = getenv("MEGATTS2_TC_HALO");          // 0: every tap re-loads its activation tile (the plain form)
-    const char* be = getenv("MEGATTS2_TC_HALO_BO");       // 1: base-offset field set in the row-shifted descriptors (diagnostics)
-    e.halo = !(he && he[0] == '0');
-    e.halo_bo = be ? atoi(be) : 0;
-    const char* hp = getenv("MEGATTS2_TC_HALO_PAIR");
-    e.halo_pair = hp ? atoi(hp) : 1;          // 0 off, 1 = the C = 64 stage only (default), 2 = C = 32 too
-    // dense-layer dispatch: 0 = tile width by grid fill (rounds 1-2), 1 = tile width by modelled cost (default), 2 = tile
-    // width, K split and pairing all by modelled cost (experimental: measured equal to 1 overall, see conv_tc())
-    const char* mo = getenv("MEGATTS2_TC_MODEL");
-    e.model = mo ? atoi(mo) : 1;
-    return e;
-  }();
-  return env;
 }
 
 struct CMapKey {
@@ -933,9 +869,7 @@ static int conv_tc_launch(const ConvTcMaps& maps, const ConvTcArgs& a, cudaStrea
 
 template <int NP>
 static int conv_tc_dispatch(const ConvTcMaps& maps, const ConvTcArgs& a, int BN, int SWB, bool pair, cudaStream_t st) {
-  if (pair) return SWB == 128 ? conv_tc_launch<128, 128, 1, NP>(maps, a, st) : conv_tc_launch<128, 64, 1, NP>(maps, a, st);
-  if (SWB == 64 && BN == 128) return conv_tc_launch<128, 64, 0, NP>(maps, a, st);
-  if (SWB == 64 && BN == 64) return conv_tc_launch<64, 64, 0, NP>(maps, a, st);
+  if (pair) return conv_tc_launch<128, 128, 1, NP>(maps, a, st);
   if (SWB == 64) return conv_tc_launch<32, 64, 0, NP>(maps, a, st);
   if (BN == 128) return conv_tc_launch<128, 128, 0, NP>(maps, a, st);
   if (BN == 64) return conv_tc_launch<64, 128, 0, NP>(maps, a, st);
@@ -973,125 +907,90 @@ bool conv_tc_eligible(const mtts_conv_params& p) {
   return 3 * rows * p.Cin * 2 + 2048 <= p.tc_scratch_bytes;
 }
 
-// The launch plan of one tap-GEMM: K-slab width, N-tile width, K splits, CTA pairing, halo form.  A pure function of the shape,
-// the SM budget and the (read-once) tuning switches, so the policy can be queried and tested without a GPU
-// (mtts_tc_plan_query, tests/test_abi_and_host.py).
+// Split-K cost model (cycles per CTA): at most CTC_SPLITK_MAX splits, taken when the split walk plus its reduction costs less
+// than CTC_SPLITK_MARGIN of the unsplit walk.  A reduction that REPLACES the LayerNorm launch that would follow anyway
+// (tc_splitk_reduce_ln_kernel) is modelled at 2000 cycles instead of the plain reduction's 9000: that makes the out-projection /
+// FF2 layers split up to steps 18 (PLM) / 24 (ADM), and every affected step got faster, PLM -0.4 ms, ADM -1.0 ms per decode
+// (profiles/r3c_splitk_constants.log, r3d_lncost_curves.log)
+constexpr int CTC_SPLITK_MAX = 8;
+constexpr double CTC_SPLITK_MARGIN = 0.85;
+constexpr double CTC_REDUCE_CYCLES = 9000.0, CTC_REDUCE_LN_CYCLES = 2000.0;
+
+// The launch plan of one tap-GEMM: K-slab width, N-tile width, K splits, CTA pairing, halo form.  A pure function of the shape
+// and the SM count, so the policy can be queried and tested without a GPU (mtts_tc_plan_query, tests/test_abi_and_host.py).
 struct TcPlan { int SWB, BN, splits; bool pair, halo_form, halo_pair; };
-static TcPlan tc_plan(const CtcEnv& env, int sms, const mtts_conv_params& p, int np, bool ln_rides) {
+static TcPlan tc_plan(int sms, const mtts_conv_params& p, int np, bool ln_rides) {
   const int halo = p.dil * (p.k - 1);
-  int SWB = p.Cin >= 64 ? 128 : 64;
+  const int SWB = p.Cin >= 64 ? 128 : 64;
   int BN = 32;
   int splits = 1;
   bool pair = false;
-  const bool pairs_ok = env.pair_mode && !g_pairs_off;
-  if (env.model >= 2 && p.k == 1 && SWB == 128 && !env.swb64) {
-    // EXPERIMENTAL (MEGATTS2_TC_MODEL=2): tile width, K split and CTA pairing of a dense layer chosen together by modelled
-    // launch cost.  A persistent CTA walks ceil(items / SMs) work items of ceil(nk / sk) K-slabs each; a slab is 4 k-steps x
-    // 3 | 6 MMAs at 65 cycles (N = 128) or 55 (the per-instruction floor, N <= 64: tools/microbench/mma_floor2.cu).  Measured
-    // per AR step against the fill heuristics (gpurun call TM, profiles/r2tm_ar_curves.log): -0.25 ms on PLM steps 19 ... 28
-    // (which mode 1 below keeps), but +0.06 ... 0.11 ms on steps 9 ... 14, where it prefers 64-wide tiles to a 3-way K split
-    // whose reduction rides on the LayerNorm launch, and +0.02 ... 0.06 ms on steps 45 ... 54 (2-way split of FF2): the model
-    // underrates wide-tile splits.  Split-K partial sums are added in split order, so results never depend on timing.
-    const int64_t rows = (int64_t)p.B * p.Tout;
-    const int64_t mt = (int64_t)p.B * cdiv64(p.Tout, 128), mt2 = (int64_t)p.B * cdiv64(p.Tout, 256);
-    const int nk = (p.Cin + 63) / 64;
-    const double mm = 4.0 * (np == 2 ? 3 : 6);                       // MMAs per 64-wide K-slab
-    double best = 1e30;
+  // N-tile width.  Dense layers (k = 1): a persistent CTA walks ceil(tiles / SMs) tiles of nk K-slabs; a slab's MMAs cost 65
+  // cycles each at N = 128 and 55 (the per-instruction floor) at N <= 64, so the width with the cheapest walk wins and ties go
+  // to the narrower tile (under-filled grids are latency-bound: more SMs stream the weights).  The earlier rule - the widest
+  // tile that still gives 80 % of the SMs a tile - ran e.g. the PLM FF2 layer of steps 19 ... 28 as 160 tiles of N = 64 on
+  // 148 SMs, two waves, where 80 tiles of N = 128 take one: -0.25 ms per step there, -0.03 ms on ADM steps 25 ... 38
+  // (profiles/r2tm_ar_curves.log).  Convolutions (k > 1) keep that fill rule: their grids are hundreds of waves deep and the
+  // halo form wants BN == Cout.
+  if (SWB == 128) {
+    const int64_t mt = (int64_t)p.B * cdiv64(p.Tout, 128);
     const int cands[3] = {128, 64, 32};
-    for (int i = 0; i < 3; ++i) {
-      if (cands[i] > p.Cout) continue;
-      const double c = (double)cdiv64(mt * cdiv64(p.Cout, cands[i]), sms) * nk * mm * (cands[i] == 128 ? 65.0 : 55.0);
-      if (c <= best) { best = c; BN = cands[i]; }      // ties (same number of waves at the 55-cycle floor) go to the narrower
-    }                                                   // tile: more SMs stream the weights
-    if (pairs_ok && sms >= 2 && p.Cout % 128 == 0) {
-      // a pair runs 256 rows per item in the time a single CTA runs 128 (each SM's tensor core does its own half); it reads a
-      // quarter fewer operand bytes per FLOP (+1..3 % measured on full grids), so it wins ties against single CTAs
-      const double c = 0.98 * (double)cdiv64(mt2 * (p.Cout / 128), sms / 2) * nk * mm * 65.0;
-      if (c <= best) { best = c; BN = 128; pair = true; }
-    }
-    if (env.splitk && p.out_shift == 0 && p.tc_partial && p.Cout >= 128) {
-            const int64_t t128 = mt * cdiv64(p.Cout, 128);
-      for (int sk = 2; sk <= env.sk_max && sk <= nk / 2; ++sk) {
-        if ((int64_t)sk * rows * p.Cout * 4 > p.tc_partial_bytes) break;
-        // + the reduction: its own launch (~4 us) unless it replaces the LayerNorm launch (~1 us extra), + the partial sums
-        // written and read back through L2 (~4 TB/s, writes counted half)
-        const double red = (ln_rides ? 1800.0 : 7300.0) + (double)sk * rows * p.Cout * 4.0 * 6.9e-4;
-        const double c = (double)cdiv64(t128 * sk, sms) * (double)cdiv64(nk, sk) * mm * 65.0 + red;
-        if (c < best) { best = c; BN = 128; pair = false; splits = sk; }
+    if (p.k == 1) {
+      int64_t best = INT64_MAX;
+      for (int i = 0; i < 3; ++i) {
+        if (cands[i] > p.Cout) continue;
+        const int64_t c = cdiv64(mt * cdiv64(p.Cout, cands[i]), sms) * (cands[i] == 128 ? 65 : 55);
+        if (c <= best) { best = c; BN = cands[i]; }
       }
-    }
-    if (pair && (env.pair_mode == 2 || env.pair_mode == 4)) SWB = 64;      // 32-wide K-slabs (diagnostics)
-  } else {
-    // N-tile width.  A persistent CTA walks ceil(tiles / SMs) tiles of nk K-slabs; a slab's MMAs cost 65 cycles each at
-    // N = 128 and 55 (the per-instruction floor) at N <= 64, so the width with the cheapest walk wins and ties go to the
-    // narrower tile (under-filled grids are latency-bound: more SMs stream the weights).  The earlier rule - the widest tile
-    // that still gives 80 % of the SMs a tile - ran e.g. the PLM FF2 layer of steps 19 ... 28 as 160 tiles of N = 64 on 148 SMs,
-    // two waves, where 80 tiles of N = 128 take one: -0.25 ms per step there, -0.03 ms on ADM steps 25 ... 38 (gpurun call TM,
-    // profiles/r2tm_ar_curves.log; MEGATTS2_TC_MODEL=0 restores it).  Convolutions (k > 1) keep the fill rule: their grids are
-    // hundreds of waves deep and the halo form wants BN == Cout.
-    if (SWB == 128) {
-      const int64_t mt = (int64_t)p.B * cdiv64(p.Tout, 128);
-      const int cands[3] = {128, 64, 32};
-      if (env.model >= 1 && p.k == 1) {
-        int64_t best = INT64_MAX;
-        for (int i = 0; i < 3; ++i) {
-          if (cands[i] > p.Cout) continue;
-          const int64_t c = cdiv64(mt * cdiv64(p.Cout, cands[i]), sms) * (cands[i] == 128 ? 65 : 55);
-          if (c <= best) { best = c; BN = cands[i]; }
-        }
-      } else {
-        for (int i = 0; i < 3; ++i) {
-          if (cands[i] > p.Cout) continue;
-          BN = cands[i];
-          if (mt * cdiv64(p.Cout, cands[i]) >= (int64_t)(sms * 4) / 5) break;
-        }
+    } else {
+      for (int i = 0; i < 3; ++i) {
+        if (cands[i] > p.Cout) continue;
+        BN = cands[i];
+        if (mt * cdiv64(p.Cout, cands[i]) >= (int64_t)(sms * 4) / 5) break;
       }
-    }
-    // split-K for dense layers with too few output tiles to fill the GPU (the early steps of the AR loops, the N = 1024
-    // layers up to ~30 steps): narrow tiles would pay the 55-cycle minimum per MMA (tools/microbench/mma_floor.cu) on
-    // every k-step, so K is split across CTAs at full tile width instead and a second kernel reduces the partials
-    {
-      const int64_t rows = (int64_t)p.B * p.Tout;
-      const int64_t t128 = (int64_t)p.B * cdiv64(p.Tout, 128) * cdiv64(p.Cout, 128);
-      const int nk = (p.Cin + 63) / 64;
-      if (env.splitk && SWB == 128 && p.k == 1 && p.out_shift == 0 && p.tc_partial && p.Cout >= 128 &&
-          t128 < (int64_t)(sms * 4) / 5) {
-        int sk = (int)(sms / t128);
-        if (sk > env.sk_max) sk = env.sk_max;
-        if (sk > nk / 2) sk = nk / 2;
-        if (sk >= 2 && (int64_t)sk * rows * p.Cout * 4 <= p.tc_partial_bytes) {
-          const int64_t tiles_bn = (int64_t)p.B * cdiv64(p.Tout, 128) * cdiv64(p.Cout, BN);
-          const double waves = (double)cdiv64(tiles_bn, sms);
-          const double mmas = 4.0 * (2 * np);                                                 // MMAs per 64-wide K-slab
-          const double cost_now = waves * nk * mmas * (BN == 128 ? 65.0 : 55.0);                // cycles per CTA
-          const double cost_split = (double)cdiv64(nk, sk) * mmas * 65.0 + (ln_rides ? env.ln_red : 9000.0);   // + reduction kernel
-          if (cost_split < env.margin * cost_now) { splits = sk; BN = 128; }
-        }
-      }
-    }
-    // CTA pairs (cta_group::2): two SMs share one 256 x 128 tile; each stages its own 128 activation rows and HALF of the
-    // weight tile, so a quarter fewer bytes cross L2 -> SM and a quarter fewer operand bytes are read from shared memory
-    // per FLOP.  Measured (tools/bench_tc_shapes.py): +1..3 % on the dense layers, -5 % on the ragged-T convolutions
-    // (256-row tiles waste more of the last tile), so pairs are used for k = 1 only.
-    if (env.swb64) SWB = 64;
-    if (pairs_ok && splits == 1 && BN == 128 && p.Cout % 128 == 0 && (p.k == 1 || env.pair_mode >= 3)) {
-      const int64_t t256 = (int64_t)p.B * cdiv64(p.Tout, 256) * (p.Cout / 128);
-      const double eff128 = (double)p.Tout / (128.0 * cdiv64(p.Tout, 128)), eff256 = (double)p.Tout / (256.0 * cdiv64(p.Tout, 256));
-      pair = t256 >= (int64_t)(sms / 2) * 4 / 5 && eff256 >= 0.9 * eff128;
-      if (pair && (env.pair_mode == 2 || env.pair_mode == 4)) SWB = 64;      // 32-wide K-slabs
     }
   }
+  // split-K for dense layers with too few output tiles to fill the GPU (the early steps of the AR loops, the N = 1024
+  // layers up to ~30 steps): narrow tiles would pay the 55-cycle minimum per MMA (tools/microbench/mma_floor.cu) on
+  // every k-step, so K is split across CTAs at full tile width instead and a second kernel reduces the partials
+  {
+    const int64_t rows = (int64_t)p.B * p.Tout;
+    const int64_t t128 = (int64_t)p.B * cdiv64(p.Tout, 128) * cdiv64(p.Cout, 128);
+    const int nk = (p.Cin + 63) / 64;
+    if (SWB == 128 && p.k == 1 && p.out_shift == 0 && p.tc_partial && p.Cout >= 128 && t128 < (int64_t)(sms * 4) / 5) {
+      int sk = (int)(sms / t128);
+      if (sk > CTC_SPLITK_MAX) sk = CTC_SPLITK_MAX;
+      if (sk > nk / 2) sk = nk / 2;
+      if (sk >= 2 && (int64_t)sk * rows * p.Cout * 4 <= p.tc_partial_bytes) {
+        const int64_t tiles_bn = (int64_t)p.B * cdiv64(p.Tout, 128) * cdiv64(p.Cout, BN);
+        const double waves = (double)cdiv64(tiles_bn, sms);
+        const double mmas = 4.0 * (2 * np);                                                 // MMAs per 64-wide K-slab
+        const double cost_now = waves * nk * mmas * (BN == 128 ? 65.0 : 55.0);                // cycles per CTA
+        const double cost_split = (double)cdiv64(nk, sk) * mmas * 65.0 + (ln_rides ? CTC_REDUCE_LN_CYCLES : CTC_REDUCE_CYCLES);
+        if (cost_split < CTC_SPLITK_MARGIN * cost_now) { splits = sk; BN = 128; }
+      }
+    }
+  }
+  // CTA pairs (cta_group::2): two SMs share one 256 x 128 tile; each stages its own 128 activation rows and HALF of the
+  // weight tile, so a quarter fewer bytes cross L2 -> SM and a quarter fewer operand bytes are read from shared memory
+  // per FLOP.  Measured (tools/bench_tc_shapes.py): +1..3 % on the dense layers, -5 % on the ragged-T convolutions
+  // (256-row tiles waste more of the last tile), so pairs are used for k = 1 only.
+  if (splits == 1 && BN == 128 && p.Cout % 128 == 0 && p.k == 1) {
+    const int64_t t256 = (int64_t)p.B * cdiv64(p.Tout, 256) * (p.Cout / 128);
+    const double eff128 = (double)p.Tout / (128.0 * cdiv64(p.Tout, 128)), eff256 = (double)p.Tout / (256.0 * cdiv64(p.Tout, 256));
+    pair = t256 >= (int64_t)(sms / 2) * 4 / 5 && eff256 >= 0.9 * eff128;
+  }
   // halo form: one K-slab per tap (Cin <= SWB / 2), the activation tile + halo fits the 192-row buffer
-  const bool halo_form = env.halo && !pair && splits == 1 && p.out_shift == 0 && p.k > 1 && p.Cin <= SWB / 2 &&
+  const bool halo_form = !pair && splits == 1 && p.out_shift == 0 && p.k > 1 && p.Cin <= SWB / 2 &&
                          halo + 128 <= CTC_HALO_ROWS &&   // (the halo kernel's epilogue has no K-split / transposed-conv paths)
                          ((SWB == 64 && BN == 32) || (SWB == 128 && BN == 64)) && p.Cout == BN;
   // ... as a CTA pair: an N = 32 / 64 MMA costs 41 / 48 cycles whatever its M (128 or 256: 52 cycles, measured with
   // tools/microbench/mma_floor2.cu), and these layers issue k * Cin / 16 * 3 of them per tile, so one instruction per 256
-  // rows nearly halves their tensor-pipe time.  Measured (gpurun calls R, S): C = 64, k = 7: 0.415 -> 0.358 ms; C = 32: 0.424 ->
-  // 0.453 ms (its tiles are paced by the epilogue, not by MMA issue; four accumulator buffers instead of two change nothing
-  // either: call T) - so pairs are the default for the C = 64 stage only (MEGATTS2_TC_HALO_PAIR = 0 | 1 | 2)
+  // rows nearly halves their tensor-pipe time.  Measured: C = 64, k = 7: 0.415 -> 0.358 ms; C = 32: 0.424 -> 0.453 ms (its
+  // tiles are paced by the epilogue, not by MMA issue; four accumulator buffers instead of two change nothing either:
+  // profiles/r2r_tc_shapes.log, r2s_stages_halo_pair_modes.log, r2t_nacc4_ab.log) - so pairs serve the C = 64 stage only
   bool halo_pair = false;
-  if (halo_form && !g_pairs_off && (env.halo_pair >= 2 || (env.halo_pair == 1 && SWB == 128))) {
+  if (halo_form && SWB == 128) {
     const int64_t t256 = (int64_t)p.B * cdiv64(p.Tout, 256);
     const double eff128 = (double)p.Tout / (128.0 * cdiv64(p.Tout, 128)), eff256 = (double)p.Tout / (256.0 * cdiv64(p.Tout, 256));
     halo_pair = t256 >= (int64_t)(sms / 2) * 2 && eff256 >= 0.9 * eff128;
@@ -1103,7 +1002,6 @@ static TcPlan tc_plan(const CtcEnv& env, int sms, const mtts_conv_params& p, int
 
 int conv_tc(const mtts_conv_params& p, cudaStream_t st, LnFuse* ln) {
   if (ln) ln->done = 0;
-  const CtcEnv& env = ctc_env();
   const int sms = cur_device_sms();
   const int fmt = p.tc_fmt;
   const int np = fmt == MTTS_TC_F16X2 ? 2 : 3;
@@ -1122,7 +1020,7 @@ int conv_tc(const mtts_conv_params& p, cudaStream_t st, LnFuse* ln) {
   }
   // the reduction of a split launch can carry the LayerNorm the caller asked for when a row is 3 / 4 / 6 / 8 x 128 wide
   const bool ln_rides = ln && ln->po.p && p.y && !p.tc_out_planes && (p.Cout == 1024 || p.Cout == 768 || p.Cout == 512 || p.Cout == 384);
-  const TcPlan pl = tc_plan(env, sms, p, np, ln_rides);
+  const TcPlan pl = tc_plan(sms, p, np, ln_rides);
   const int SWB = pl.SWB, BN = pl.BN, splits = pl.splits;
   const bool pair = pl.pair, halo_form = pl.halo_form, halo_pair = pl.halo_pair;
   const int b_rows = (pair || halo_pair) ? BN / 2 : BN;
@@ -1143,11 +1041,8 @@ int conv_tc(const mtts_conv_params& p, cudaStream_t st, LnFuse* ln) {
   a.op = reinterpret_cast<__nv_bfloat16*>(p.tc_out_planes); a.op_stride = p.tc_out_plane_stride; a.op_ld = p.tc_out_ld;
   a.op_tp = p.tc_out_tp; a.op_hl = p.tc_out_hl; a.op_act = p.tc_out_act; a.op_slope = p.tc_out_slope;
   a.splits = splits; a.partial = reinterpret_cast<float*>(p.tc_partial);
-  a.fmt = fmt; a.ovf = ovf; a.bo_mode = env.halo_bo; a.row0 = p.tc_in_row0;
-  if (halo_form && halo_pair) {
-    if (SWB == 64) return np == 2 ? conv_tc_launch<32, 64, 1, 2, 1>(maps, a, st) : conv_tc_launch<32, 64, 1, 3, 1>(maps, a, st);
-    return np == 2 ? conv_tc_launch<64, 128, 1, 2, 1>(maps, a, st) : conv_tc_launch<64, 128, 1, 3, 1>(maps, a, st);
-  }
+  a.fmt = fmt; a.ovf = ovf; a.row0 = p.tc_in_row0;
+  if (halo_pair) return np == 2 ? conv_tc_launch<64, 128, 1, 2, 1>(maps, a, st) : conv_tc_launch<64, 128, 1, 3, 1>(maps, a, st);
   if (halo_form) {
     if (SWB == 64) return np == 2 ? conv_tc_launch<32, 64, 0, 2, 1>(maps, a, st) : conv_tc_launch<32, 64, 0, 3, 1>(maps, a, st);
     return np == 2 ? conv_tc_launch<64, 128, 0, 2, 1>(maps, a, st) : conv_tc_launch<64, 128, 0, 3, 1>(maps, a, st);
@@ -1185,7 +1080,7 @@ int tc_plan_query(int sms, int B, int T, int Cin, int Cout, int k, int dil, int 
   static float dummy;
   p.y = &dummy;
   if (partial_bytes > 0) { p.tc_partial = &dummy; p.tc_partial_bytes = partial_bytes; }
-  const TcPlan pl = tc_plan(ctc_env(), sms, p, fmt == MTTS_TC_F16X2 ? 2 : 3, ln_rides != 0);
+  const TcPlan pl = tc_plan(sms, p, fmt == MTTS_TC_F16X2 ? 2 : 3, ln_rides != 0);
   out5[0] = pl.BN; out5[1] = pl.splits; out5[2] = pl.pair ? 1 : 0; out5[3] = pl.halo_form ? (pl.halo_pair ? 2 : 1) : 0; out5[4] = pl.SWB;
   return 0;
 }

@@ -95,24 +95,6 @@ static int lin_planes(const TcScratch* tc, __nv_bfloat16* planes, int64_t M, int
   return rc;
 }
 
-// MEGATTS2_LN_FUSE=0: LayerNorm always as its own launch (read once)
-static bool ln_fuse() {
-  static const bool on = [] {
-    const char* e = getenv("MEGATTS2_LN_FUSE");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
-// MEGATTS2_LAST_ROW_TC=0: the final layer's last-row work stays on the exact FFMA engine (read once)
-static bool last_row_tc() {
-  static const bool on = [] {
-    const char* e = getenv("MEGATTS2_LAST_ROW_TC");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
 // dense layer dispatch: one tap-GEMM call; conv1d() picks the tcgen05 engine when planes + scratch are attached
 // and the shape is eligible (M >= 128), else the exact FFMA engine
 static int lin(const mtts_encoder* e, const TcScratch* tc, const float* x, int ldx, int64_t M, int K, int N,
@@ -194,7 +176,7 @@ static int encoder_forward(const mtts_encoder* e, const float* x, float* y, int 
         MTTS_TRY(attention(ap, st));
         // out-projection (+ residual); a split-K launch's reduction kernel applies LN2 to the finished rows as well
         LnFuse ln2{L.ln2_g, L.ln2_b, 1e-5f, pa_out, 0};
-        MTTS_TRY(lin_planes(tc, Pa, M, D, D, L.w_o_tc, L.b_o, xin, D, xw, D, 0, nullptr, 0, st, part, part_bytes, ln_fuse() ? &ln2 : nullptr));
+        MTTS_TRY(lin_planes(tc, Pa, M, D, D, L.w_o_tc, L.b_o, xin, D, xw, D, 0, nullptr, 0, st, part, part_bytes, &ln2));
         if (!ln2.done) MTTS_TRY(layernorm_ex(xw, D, L.ln2_g, L.ln2_b, nullptr, 0, nullptr, 0, M, D, 1e-5f, 0, 0, pa_out, st));
         // FF1: relu(h W1 + b1) goes straight to planes P_b; FF2 reads them
         MTTS_TRY(lin_planes(tc, Pa, M, D, F, L.w_ff1_tc, L.b_ff1, nullptr, 0, nullptr, 0, MTTS_ACT_RELU, Pb, F, st, part, part_bytes));
@@ -203,7 +185,7 @@ static int encoder_forward(const mtts_encoder* e, const float* x, float* y, int 
         const bool next_ln = l + 1 < e->n_layers;
         LnFuse ln1{next_ln ? e->layers[l + 1].ln1_g : nullptr, next_ln ? e->layers[l + 1].ln1_b : nullptr, 1e-5f, pa_out, 0};
         MTTS_TRY(lin_planes(tc, Pb, M, F, D, L.w_ff2_tc, L.b_ff2, xw, D, xw, D, 0, nullptr, 0, st, part, part_bytes,
-                            (next_ln && ln_fuse()) ? &ln1 : nullptr));
+                            next_ln ? &ln1 : nullptr));
         ln1_done = ln1.done != 0;
         xin = xw;
         continue;
@@ -235,7 +217,7 @@ static int encoder_forward(const mtts_encoder* e, const float* x, float* y, int 
       // final layer, last position only (exact: nothing else is consumed downstream)
       ap.q = qkv + (int64_t)(T - 1) * 3 * D; ap.q_sb = (int64_t)T * 3 * D; ap.q_st = 3 * D; ap.Tq = 1;
       if (mask) ap.mask = mask + (int64_t)(T - 1) * mask_sq;
-      if (fused && B >= 32 && last_row_tc()) {
+      if (fused && B >= 32) {
         // the B last rows as one half-filled 128-row tile on the tensor cores (split-K fills the SMs): the attention rows,
         // LN2 and FF1 write operand planes like the full-sequence layers.  The exact-FFMA form below took 21 + 5 us per
         // dense layer at B = 64 (weight streaming through the FP32 pipe), 4 layers per AR step.
@@ -873,11 +855,6 @@ int mtts_split_planes_f32(const float* x, int32_t ldx, int64_t rows, int32_t C, 
   return split_planes(x, ldx, rows, C, planes, fmt, (cudaStream_t)stream);
 }
 int mtts_tc_overflow_bind(int32_t* flag_dev) { return tc_overflow_bind(flag_dev); }
-int mtts_set_attention_pair_min(int32_t min_len) { return set_attention_pair_min(min_len); }
-int mtts_set_sm_limit(int32_t n_sms) { return set_sm_limit(n_sms); }
-int mtts_set_launch_policy(int32_t sm_limit, int32_t allow_pairs, int32_t allow_pdl) {
-  return set_launch_policy(sm_limit, allow_pairs, allow_pdl);
-}
 int mtts_tc_plan_query(int32_t n_sms, int32_t B, int32_t T, int32_t Cin, int32_t Cout, int32_t k, int32_t dil, int32_t fmt,
                        int64_t partial_bytes, int32_t ln_rides, int32_t* out5) {
   return tc_plan_query(n_sms, B, T, Cin, Cout, k, dil, fmt, partial_bytes, ln_rides, out5);

@@ -76,8 +76,6 @@ __device__ __forceinline__ void store_planes4(__nv_bfloat16* planes, int64_t pla
 int32_t* tc_ovf_ptr();
 int cur_device();
 int cur_device_sms();
-int set_sm_limit(int n);
-int set_launch_policy(int sm_limit, int allow_pairs, int allow_pdl);
 int tc_plan_query(int sms, int B, int T, int Cin, int Cout, int k, int dil, int fmt, int64_t partial_bytes, int ln_rides, int32_t* out5);
 static inline int tc_fmt_of_engine(int engine) { return engine == 2 ? MTTS_TC_F16X2 : MTTS_TC_BF16X3; }
 int layernorm_ex(const float* x, int ldx, const float* gamma, const float* beta, const float* res, int ldr, float* y,
@@ -109,9 +107,6 @@ int layernorm(const float* x, int ldx, const float* gamma, const float* beta, co
 int attention(const mtts_attn_params& p, cudaStream_t st);
 bool attention_tc_eligible(const mtts_attn_params& p);
 int attention_tc(const mtts_attn_params& p, cudaStream_t st);
-bool attention_tc_pair_eligible(const mtts_attn_params& p);
-int attention_tc_pair(const mtts_attn_params& p, cudaStream_t st);
-int set_attention_pair_min(int n);   // tcgen05 (attn_tc.cu)
 int vq_argmin(const float* x, int ldx, const float* embed, int64_t N, int D, int K, int64_t* idx, cudaStream_t st);
 int vq_gather(const int64_t* idx, int idx_ld, const float* embed, int D, int K, int B, int T_out, int repeat, float* y,
               int64_t y_sb, int ldy, cudaStream_t st);

@@ -387,12 +387,6 @@ static int attn_launch(const mtts_attn_params& p, cudaStream_t st) {
   return 0;
 }
 
-static std::atomic<int> g_attn_pair_min{[] {
-  const char* m = getenv("MEGATTS2_ATTN_PAIR_MIN");
-  return m ? atoi(m) : (1 << 30);
-}()};
-int set_attention_pair_min(int n) { return g_attn_pair_min.exchange(n > 0 ? n : (1 << 30), std::memory_order_relaxed); }
-
 int attention(const mtts_attn_params& p, cudaStream_t st) {
   MTTS_REQUIRE(p.q && p.k && p.v && (p.o || p.o_planes), "null pointer");
   MTTS_REQUIRE(!p.o_planes || (p.o_planes_ld % 4 == 0 && p.o_plane_stride % 4 == 0), "plane output alignment");
@@ -403,24 +397,7 @@ int attention(const mtts_attn_params& p, cudaStream_t st) {
   // the C4 step shapes (Tq = Tk <= 64, profiles/r2c_attention_tc_ab.md) the phase-serialised tensor-core kernel is 1.5x
   // SLOWER than this fp32 kernel (58 vs 38 us per launch: the problem is 64 x 64 x 64 per head, all latency), so the AR
   // steps of the benchmark stay here; longer sequences (teacher-forced forwards, config C3) go to the tensor cores.
-  // (MEGATTS2_ATTN_TC = 0 disables it, MEGATTS2_ATTN_TC_MIN sets the minimum Tq; read once per process)
-  {
-    static const int tc_min = [] {
-      const char* e = getenv("MEGATTS2_ATTN_TC");
-      if (e && e[0] == '0') return 1 << 30;
-      const char* m = getenv("MEGATTS2_ATTN_TC_MIN");
-      return m ? atoi(m) : 65;
-    }();
-    if (p.Tq >= tc_min && attention_tc_eligible(p)) return attention_tc(p, st);
-    // AR steps (Tq == Tk <= 64): two heads stacked into one 128-row tile (attn_tc_pair_kernel).  Measured (gpurun call Q,
-    // profiles/r2q_attention_pair_ab.log): in isolation 39.6 vs 52.8 us at S = 64 and 31.0 vs 39.4 us at S = 48 for the PLM
-    // heads, level for the ADM heads (dh 96: one CTA per SM), slower below S = 40; inside the step it LOSES (PLM 151.8 ->
-    // 154.3 ms, ADM 56.3 -> 64.4 ms): the operand conversions, not the MMAs, are what a 64 x 64 x 64 head costs, and its
-    // 97-144 KB / 256 TMEM columns keep the neighbouring GEMMs' CTAs from overlapping.  So it is opt-in
-    // (mtts_set_attention_pair_min / MEGATTS2_ATTN_PAIR_MIN: shortest sequence that takes it), off by default.
-    const int pair_min = g_attn_pair_min.load(std::memory_order_relaxed);
-    if (p.Tq >= pair_min && attention_tc_pair_eligible(p)) return attention_tc_pair(p, st);
-  }
+  if (p.Tq >= 65 && attention_tc_eligible(p)) return attention_tc(p, st);
   // dh <= 128: one CTA of 8 warps covers a whole AR-step sequence (Tq <= 64), so K and V are read once per (b, h);
   // the rows are dealt evenly to the warps (RW = ceil(Tq / 8) rows each) - with a fixed 8 rows per warp a 35-row
   // step left three of the eight warps idle.  Row results do not depend on RW (each row's sums keep their order).

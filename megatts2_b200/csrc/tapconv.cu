@@ -419,7 +419,7 @@ int conv1d_ffma(const mtts_conv_params& p, cudaStream_t st) {
     if (p.k == 1 && p.stride == 1 && p.pad == 0 && p.out_shift == 0 && !p.in_lens && M <= 256 && tiles64 <= 148 &&
         nk >= 16 && p.tc_scratch) {
       // two CTAs per SM: a lone 8-warp CTA cannot hide the L2 latency of its one-chunk-ahead prefetch
-      static const int target = []() { const char* e = getenv("MEGATTS2_SPLITK_CTAS"); return e ? atoi(e) : 296; }();
+      constexpr int target = 296;
       int splits = (int)(target / tiles64);
       if (splits > 16) splits = 16;
       if (splits > nk / 4) splits = nk / 4;

@@ -182,12 +182,10 @@ __device__ __forceinline__ void tc_commit_2sm_l(uint32_t bar, uint32_t leader) {
       : "memory");
 }
 
-// descriptor of an operand whose start address is shifted by whole rows inside a swizzled tile: low word = address,
-// base offset (bits 49..51) = the row phase of the start address inside the 8-row swizzle pattern
-__device__ __forceinline__ uint64_t umma_desc_shifted(uint64_t desc_base, uint32_t smem_addr, int bo_mode) {
-  uint64_t d = desc_base | (uint64_t)((smem_addr >> 4) & 0x3FFF);
-  if (bo_mode) d |= (uint64_t)((smem_addr >> 7) & 7) << 49;
-  return d;
+// descriptor of an operand whose start address is shifted by whole rows inside a swizzled tile: low word = address, base
+// offset left at zero (the swizzle follows the address bits, conv_tc.cu)
+__device__ __forceinline__ uint64_t umma_desc_shifted(uint64_t desc_base, uint32_t smem_addr) {
+  return desc_base | (uint64_t)((smem_addr >> 4) & 0x3FFF);
 }
 
 // One tap of the f16x2 halo form: NKS k-steps x three MMAs (x1 w2' and x2' w1 into the correction accumulator, x1 w1 into

@@ -158,8 +158,7 @@ class MegaPLM(pack.PlanMixin, nn.Module):
             return (codes, logits) if return_logits else (codes,)
 
         # the whole decode is one device-side enqueue sequence: replayed as a CUDA graph from the second call on
-        out = self._graphs().run(("plm", pl.serial, B, T, bool(return_logits), tc.stride(0), tc.stride(1),
-                                  ops.launch_policy_now()), (tc,), run)
+        out = self._graphs().run(("plm", pl.serial, B, T, bool(return_logits), tc.stride(0), tc.stride(1)), (tc,), run)
         codes = out[0]
         logits = out[1] if return_logits else None
         return (codes, logits) if return_logits else codes
@@ -272,8 +271,7 @@ class MegaADM(pack.PlanMixin, nn.Module):
                                            ws.data_ptr(), ws.numel(), ops._stream()))
             return (dur, raw) if return_raw else (dur,)
 
-        out = self._graphs().run(("adm", pl.serial, B, T, bool(return_raw), tc.stride(0), tc.stride(1),
-                                  ops.launch_policy_now()), (tc,), run)
+        out = self._graphs().run(("adm", pl.serial, B, T, bool(return_raw), tc.stride(0), tc.stride(1)), (tc,), run)
         dur = out[0]
         raw = out[1] if return_raw else None
         dur = dur.unsqueeze(-1)
@@ -309,11 +307,6 @@ class MegaADM(pack.PlanMixin, nn.Module):
 
 
 # ------------------------------------------------------------------------------------------
-# Overlapped prompt re-vocode (Megatts._synthesize): defaults of MEGATTS2_REVOCODE_SMS / _FRAC / _FROM
-REVOCODE_SMS_DEFAULT = 0
-REVOCODE_FRAC_DEFAULT = 1.0
-REVOCODE_FROM_DEFAULT = "mrte"
-
 HIFIGAN_V1 = dict(in_channels=80, upsample_initial_channel=512, upsample_factors=(8, 8, 2, 2),
                   upsample_kernel_sizes=(16, 16, 4, 4), resblock_kernel_sizes=(3, 7, 11),
                   resblock_dilation_sizes=((1, 3, 5), (1, 3, 5), (1, 3, 5)), inference_padding=5)
@@ -530,73 +523,29 @@ class Megatts(nn.Module):
         ``return_lengths``: also return the valid sample count per utterance (prompt part included).
         ``causal_decode=True`` swaps both AR loops for the opt-in causal KV-cache decode (training semantics; NOT the
         reference's infer() - different ids; SURVEY.md 8f-1).
-        ``overlap_prompt``: the prompt re-vocode runs on a side stream with an SM budget (MEGATTS2_REVOCODE_SMS) beside the
-        MRTE + ADM stages, which get the remaining SMs (see ``_synthesize``); False forces the sequential form, True the
-        overlapped one even when the budget's default is 0.  Waveforms are identical either way (the vocoder has no
-        batch- or grid-dependent reduction order); the ADM / MRTE dense layers pick their K split from the SM budget, so
-        their fp32 results move within rounding noise.
+        ``overlap_prompt``: None or False; the prompt re-vocode runs after the synthesis on the calling stream.  Running it
+        on a side stream beside MRTE + ADM measured no faster and was removed, so True raises ``ValueError``.
         ``check_range``: with the f16x2 operand engine, read the range flag after the batch (one 4-byte readback) and,
         if any activation left the fp16 range, redo the batch on the bf16x3 engine."""
+        if overlap_prompt:
+            raise ValueError("overlap_prompt=True is not supported: the prompt re-vocode runs after the synthesis")
         dev = phone_tokens.device
-        out = self._synthesize(phone_tokens, mels, forced_durations, causal_decode, prompt_mels, overlap_prompt)
+        out = self._synthesize(phone_tokens, mels, forced_durations, causal_decode, prompt_mels)
         if check_range and pack.default_engine() == pack.ENGINE_F16X2 and ops.tc_overflow(dev):
             import warnings
             warnings.warn("megatts2_b200: an activation left the fp16 range of the f16x2 operand split; "
                           "re-running this batch on the bf16x3 engine")
             with pack.engine_scope(pack.ENGINE_BF16X3):
-                out = self._synthesize(phone_tokens, mels, forced_durations, causal_decode, prompt_mels, overlap_prompt)
+                out = self._synthesize(phone_tokens, mels, forced_durations, causal_decode, prompt_mels)
         if return_intermediates:
             return out
         return (out["wav"], out["wav_lens"]) if return_lengths else out["wav"]
 
-    def _revocode_cfg(self):
-        """(V, frac, start) of the overlapped prompt re-vocode: V = SM budget of the side stream (MEGATTS2_REVOCODE_SMS; 0 = run
-        the re-vocode after the synthesis on the calling stream), frac = share of the batch's prompts re-vocoded there
-        (MEGATTS2_REVOCODE_FRAC; the rest follows sequentially at full width), start = 'mrte' | 'adm': the first stage of the
-        calling stream that runs beside it, on the remaining SMs (MEGATTS2_REVOCODE_FROM)."""
-        import os
-        return (int(os.environ.get("MEGATTS2_REVOCODE_SMS", str(REVOCODE_SMS_DEFAULT))),
-                float(os.environ.get("MEGATTS2_REVOCODE_FRAC", str(REVOCODE_FRAC_DEFAULT))),
-                os.environ.get("MEGATTS2_REVOCODE_FROM", REVOCODE_FROM_DEFAULT))
-
-    def _synthesize(self, phone_tokens, mels, forced_durations, causal_decode, prompt_mels, overlap_prompt=None):
-        # The prompt re-vocode (:371-372) depends on nothing the synthesis computes, and the ADM loop (latency-bound: ~4 k short
-        # dependent launches that fill a fraction of the SMs) leaves most of the device idle: the re-vocode is enqueued first,
-        # on a side stream with an SM budget of V, and MRTE + ADM run beside it on the other SMs.  ops.launch_policy carries
-        # the three rules that make two streams share the device (csrc/conv_tc.cu, set_launch_policy): complementary budgets,
-        # no programmatic dependent launch on the vocoder's stream, no CTA pairs on the AR stream.  The calling stream joins
-        # the side stream before the first full-width stage (length regulator -> PLM), so nothing sized for the whole device is
-        # ever enqueued while the vocoder's persistent CTAs hold SMs.
-        pw_side, side, n_side = None, None, 0
-        V, frac, start = self._revocode_cfg()
-        dev = phone_tokens.device
-        overlap = prompt_mels is not None and overlap_prompt is not False and (V > 0 or overlap_prompt is True)
+    def _synthesize(self, phone_tokens, mels, forced_durations, causal_decode, prompt_mels):
         adm_decode = self.adm.infer_causal if causal_decode else self.adm.infer
         plm_decode = self.plm.infer_causal if causal_decode else self.plm.infer
-        if overlap:
-            nsm = ops.sm_count(dev)
-            V = max(8, min(V if V > 0 else (2 * nsm) // 3, nsm - 8))
-            n_side = max(1, min(prompt_mels.shape[0], int(round(prompt_mels.shape[0] * frac))))
-            self.hifi_gan.generator._plan_get()          # weights are packed on the calling stream, before the fork
-            main = torch.cuda.current_stream(dev)
-            if getattr(self, "_side_stream", None) is None:
-                self._side_stream = torch.cuda.Stream(device=dev)
-            side = self._side_stream
-            if start == "adm":
-                tc_latent = self.generator.mrte.tc_latent(phone_tokens, mels)
-            side.wait_stream(main)
-            prompt_mels.record_stream(side)
-            with torch.cuda.stream(side), ops.launch_policy(V, pairs=True, pdl=False):
-                pw_side = self.hifi_gan.decode_batch_cl(prompt_mels[:n_side])
-            with ops.launch_policy(nsm - V, pairs=False, pdl=True):
-                if start != "adm":
-                    tc_latent = self.generator.mrte.tc_latent(phone_tokens, mels)
-                dt = adm_decode(tc_latent)[..., 0]
-            main.wait_stream(side)
-            pw_side.record_stream(main)
-        else:
-            tc_latent = self.generator.mrte.tc_latent(phone_tokens, mels)
-            dt = adm_decode(tc_latent)[..., 0]
+        tc_latent = self.generator.mrte.tc_latent(phone_tokens, mels)
+        dt = adm_decode(tc_latent)[..., 0]
         d_used = dt if forced_durations is None else forced_durations.to(dt.device, torch.int32)
         tc_expand, totals = ops.length_regulate(tc_latent, d_used, return_host_totals=True)   # one host sync
         tc8 = ops.maxpool_time(tc_expand, 8)
@@ -621,12 +570,7 @@ class Megatts(nn.Module):
                 wav[idx, :, :wg.shape[-1]] = wg
         wav_lens = [hop * (t + 2 * pad) for t in totals]
         if prompt_mels is not None:
-            if pw_side is None:
-                pw = self.hifi_gan.decode_batch_cl(prompt_mels)       # (B, 1, hop*(Tq + 2 pad))   (:371-372)
-            elif n_side < prompt_mels.shape[0]:
-                pw = torch.cat([pw_side, self.hifi_gan.decode_batch_cl(prompt_mels[n_side:])], dim=0)
-            else:
-                pw = pw_side
+            pw = self.hifi_gan.decode_batch_cl(prompt_mels)           # (B, 1, hop*(Tq + 2 pad))   (:371-372)
             wav = torch.cat([pw, wav], dim=-1)                        # (:373)
             wav_lens = [n + pw.shape[-1] for n in wav_lens]
         return dict(tc_latent=tc_latent, dt=dt, tc_latent_expand=tc_expand, tc8=tc8, p_codes=p_codes,

@@ -7,7 +7,6 @@ convert at their boundary.
 """
 import ctypes as C
 import math
-import threading
 
 import torch
 
@@ -324,12 +323,6 @@ def _dev_index(device):
     return torch.cuda.current_device() if device.index is None else device.index
 
 
-def set_attention_pair_min(min_len):
-    """Opt-in two-heads-per-CTA tensor-core attention for AR steps of at least ``min_len`` rows (0 / None: off).
-    Returns the previous setting."""
-    return int(L.lib().mtts_set_attention_pair_min(int(min_len or 0)))
-
-
 def tc_overflow_bind(device):
     """Registers (once per device) the int32 flag the f16x2 operand split raises when an activation leaves the
     fp16 range (|x| > 65504); returns the flag tensor."""
@@ -370,40 +363,6 @@ def workspace(nbytes, device):
         assert buf.data_ptr() % 256 == 0
         _ws_cache[key] = buf
     return buf
-
-
-# ------------------------------------------------------------------------------ launch policy
-_tls = threading.local()      # the C side keeps the policy per host thread (thread_local), so does this mirror
-
-
-def launch_policy_now():
-    """(SM budget, CTA pairs allowed, PDL allowed) of the calling thread's launches; (0, 1, 1) = defaults.  Part of the
-    CUDA-graph keys: a captured graph has its grid sizes baked in."""
-    return getattr(_tls, "policy", (0, 1, 1))
-
-
-class launch_policy:
-    """``with ops.launch_policy(sm_limit, pairs=..., pdl=...)``: the enclosed enqueues of this thread size their persistent
-    grids for ``sm_limit`` SMs, optionally without CTA pairs / programmatic dependent launch (include/megatts2_b200.h,
-    mtts_set_launch_policy).  Restored on exit, also when the body raises."""
-
-    def __init__(self, sm_limit, pairs=True, pdl=True):
-        self.new = (int(sm_limit), int(bool(pairs)), int(bool(pdl)))
-
-    def __enter__(self):
-        self.old = launch_policy_now()
-        L.check(L.lib().mtts_set_launch_policy(*self.new))
-        _tls.policy = self.new
-        return self
-
-    def __exit__(self, *exc):
-        L.lib().mtts_set_launch_policy(*self.old)
-        _tls.policy = self.old
-        return False
-
-
-def sm_count(device):
-    return torch.cuda.get_device_properties(device).multi_processor_count
 
 
 def _lib_launch_count():

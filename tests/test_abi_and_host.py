@@ -20,7 +20,7 @@ def _header_symbols():
     return sorted(set(re.findall(r"\b(mtts_[a-z0-9_]+)\s*\(", txt)))
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_abi4():
     from megatts2_b200 import _lib as L
     lib = L.lib()
     syms = _header_symbols()
@@ -30,7 +30,7 @@ def test_library_exports_every_declared_symbol():
         assert hasattr(raw, s), f"missing export {s}"
         assert s in L.SIGNATURES, f"{s} has no ctypes signature"
     assert set(L.SIGNATURES) == set(syms)
-    assert lib.mtts_abi_version() == L.ABI_VERSION == 3
+    assert lib.mtts_abi_version() == L.ABI_VERSION == 4
     assert lib.mtts_launch_count() == 0
 
 
@@ -43,25 +43,6 @@ def test_error_reporting_without_gpu():
         L.check(lib.mtts_attention_f32(None, None))
 
 
-def test_launch_policy_is_scoped_and_restored():
-    """ops.launch_policy (SM budget, CTA pairs, PDL of the calling thread's launches; host state only, no CUDA call): nests,
-    restores on exit and on exceptions, and is part of the CUDA-graph keys of the AR drivers."""
-    from megatts2_b200 import ops
-    assert ops.launch_policy_now() == (0, 1, 1)
-    with ops.launch_policy(100, pairs=True, pdl=False):
-        assert ops.launch_policy_now() == (100, 1, 0)
-        with ops.launch_policy(48, pairs=False):
-            assert ops.launch_policy_now() == (48, 0, 1)
-        assert ops.launch_policy_now() == (100, 1, 0)
-    assert ops.launch_policy_now() == (0, 1, 1)
-    with pytest.raises(RuntimeError):
-        with ops.launch_policy(64):
-            raise RuntimeError("boom")
-    assert ops.launch_policy_now() == (0, 1, 1)
-    src = open(os.path.join(ROOT, "megatts2_b200", "models", "megatts2.py")).read()
-    assert src.count("ops.launch_policy_now()") >= 2          # MegaPLM.infer and MegaADM.infer graph keys
-
-
 def _plan(M, K, N, ln=0, k=1, B=1, dil=1, partial=64 << 20, sms=148):
     from megatts2_b200 import _lib as L
     out = (ctypes.c_int32 * 5)()
@@ -69,11 +50,10 @@ def _plan(M, K, N, ln=0, k=1, B=1, dil=1, partial=64 << 20, sms=148):
     return dict(BN=out[0], splits=out[1], pair=out[2], halo=out[3], swb=out[4])
 
 
-def test_tap_gemm_launch_plan_policy():
+def test_tap_gemm_launch_plan_default_policy():
     """The dispatcher's plan is a pure host function (csrc/conv_tc.cu tc_plan): dense-layer tile widths minimise
     ceil(tiles / SMs) x per-MMA cost (65 cycles at N = 128, 55 below; ties to the narrower tile), splits need partial-sum
-    space, the small-channel vocoder convs take the halo form (C = 64 as a CTA pair), and a no-pairs launch policy is obeyed."""
-    from megatts2_b200 import ops
+    space, and the small-channel vocoder convs take the halo form (C = 64 as a CTA pair)."""
     sms = 148
     cd = lambda a, b: (a + b - 1) // b
     for D, FF in ((1024, 4096), (768, 1024)):                       # PLM / ADM stacks, rows = 64 x step
@@ -93,10 +73,7 @@ def test_tap_gemm_launch_plan_policy():
                 assert _plan(M, K, N, ln, partial=0)["splits"] == 1
     # the case the fill rule got wrong: PLM FF2 at step 20 = 80 tiles of N = 128 in one wave, not 160 of N = 64 in two
     assert _plan(64 * 20, 4096, 1024, 1)["BN"] == 128
-    # full-width dense layers run as CTA pairs; not under a no-pairs policy (two streams sharing the device)
-    assert _plan(4096, 1024, 3072)["pair"] == 1
-    with ops.launch_policy(74, pairs=False):
-        assert _plan(4096, 1024, 3072, sms=74)["pair"] == 0
+    # full-width dense layers run as CTA pairs
     assert _plan(4096, 1024, 3072)["pair"] == 1
     # vocoder ResBlock convs: halo form at C = 32 (64-byte K-slabs) and C = 64 (as a pair), plain form at C = 128
     assert _plan(66816, 32, 32, k=7, B=64, dil=3, partial=0) == dict(BN=32, splits=1, pair=0, halo=1, swb=64)

@@ -5,7 +5,6 @@ Bars: integer outputs (VQ codes, PLM ids, durations, gather indices) bit-exact; 
 point within the tolerance written next to each check (fp32 vs fp32 with different
 summation order; the noise floors are in SURVEY.md §7.2)."""
 import math
-import os
 
 import numpy as np
 import pytest
@@ -197,17 +196,11 @@ def test_layernorm(C_):
                                         (16, 64, 1, 200), (4, 128, 17, 65),
                                         # tensor-core path (attn_tc.cu): one / several query tiles and key tiles, ragged edges
                                         (16, 64, 64, 64), (16, 64, 130, 300), (8, 96, 200, 200), (8, 96, 16, 16), (2, 128, 129, 64),
-                                        # two heads per CTA (AR steps, Tq == Tk <= 64)
+                                        # AR-step shapes (Tq == Tk <= 64)
                                         (16, 64, 24, 24), (16, 64, 47, 47), (8, 96, 64, 64), (2, 64, 40, 40)])
-def test_attention(H, dh, Tq, Tk):
+def test_attention_default_dispatch(H, dh, Tq, Tk):
     from megatts2_b200 import ops
-    prev = ops.set_attention_pair_min(16)     # the opt-in two-heads-per-CTA kernel takes the eligible cases
-    try:
-        _attention_cases(ops, H, dh, Tq, Tk)
-    finally:
-        ops.set_attention_pair_min(0 if prev >= (1 << 30) else prev)
-    if Tq == Tk and Tk <= 64 and H % 2 == 0 and dh in (64, 96):
-        _attention_cases(ops, H, dh, Tq, Tk)  # and the default (fp32) kernel
+    _attention_cases(ops, H, dh, Tq, Tk)
 
 
 def _attention_cases(ops, H, dh, Tq, Tk):
@@ -489,6 +482,10 @@ def test_prompt_revocode_and_synthesize_many(weights_cpu):
     assert pw.shape[-1] == 256 * (48 + 10) and both.shape[-1] == pw.shape[-1] + plain.shape[-1]
     assert torch.equal(both[..., :pw.shape[-1]], pw) and torch.equal(both[..., pw.shape[-1]:], plain)
     assert lens == [pw.shape[-1] + 256 * (11 + 10)] * 2
+    # the re-vocode always runs in line: overlap_prompt=False is the same call, True is rejected
+    assert torch.equal(tts.synthesize(phone, melp, forced_durations=forced, prompt_mels=melp, overlap_prompt=False), both)
+    with pytest.raises(ValueError, match="overlap_prompt"):
+        tts.synthesize(phone, melp, forced_durations=forced, prompt_mels=melp, overlap_prompt=True)
     # ragged front door: three utterances in two buckets, results in input order
     p2 = torch.randint(0, 320, (4,), generator=gen(46)).to(DEV)
     m2 = (torch.randn(40, 80, generator=gen(47)) * 2 - 4).to(DEV)
@@ -501,39 +498,6 @@ def test_prompt_revocode_and_synthesize_many(weights_cpu):
     w = tts.hifi_gan.decode_batch(melp.transpose(1, 2), mel_lens=torch.tensor([48, 30]), hop_len=256)
     assert float(w[1, :, 30 * 256:].abs().max()) == 0.0 and float(w[1, :, :30 * 256].abs().max()) > 0
     assert torch.equal(w[0, :, :48 * 256], pw[0, :, :48 * 256]) and float(w[0, :, 48 * 256:].abs().max()) == 0.0
-
-
-def test_overlapped_prompt_revocode(weights_cpu):
-    """Megatts._synthesize with the prompt re-vocode on a side stream (SM budget V) beside MRTE + ADM on the remaining SMs
-    (ops.launch_policy: complementary budgets, no PDL on the vocoder's stream, no CTA pairs on the AR stream): the waveform of
-    the prompt is bit-identical to the sequential form, ids / durations equal, through eager, capture and replay passes; the
-    policy is restored afterwards."""
-    from megatts2_b200 import ops
-    tts = helpers.build_megatts(weights_cpu("g"), weights_cpu("plm"), weights_cpu("adm"), weights_cpu("hifigan"), DEV)
-    B, Tp, Tm = 6, 24, 64
-    phone = torch.randint(0, 320, (B, Tp), generator=gen(71)).to(DEV)
-    melp = (torch.randn(B, Tm, 80, generator=gen(72)) * 2 - 4).to(DEV)
-    forced = torch.randint(1, 4, (B, Tp), generator=gen(73)).to(torch.int32)
-    forced[:, -1] += (forced.sum(1).max() - forced.sum(1)).to(torch.int32)          # equal totals: one vocoder group
-    forced = forced.to(DEV)
-    seq = tts.synthesize(phone, melp, forced_durations=forced, prompt_mels=melp, return_intermediates=True, overlap_prompt=False)
-    n_p = 256 * (Tm + 10)
-    keys = ("MEGATTS2_REVOCODE_SMS", "MEGATTS2_REVOCODE_FRAC", "MEGATTS2_REVOCODE_FROM")
-    saved = {k: os.environ.get(k) for k in keys}
-    try:
-        for sms, frac, start in (("100", "1.0", "mrte"), ("116", "0.5", "adm"), ("0", "1.0", "mrte")):
-            os.environ.update({keys[0]: sms, keys[1]: frac, keys[2]: start})
-            for _ in range(3):      # eager, graph capture, replay
-                ov = tts.synthesize(phone, melp, forced_durations=forced, prompt_mels=melp, return_intermediates=True,
-                                    overlap_prompt=True)
-                assert ops.launch_policy_now() == (0, 1, 1)
-                assert torch.equal(ov["wav"][..., :n_p], seq["wav"][..., :n_p])
-                assert torch.equal(ov["dt"], seq["dt"]) and torch.equal(ov["p_codes"], seq["p_codes"])
-                assert maxerr(ov["tc_latent"], seq["tc_latent"]) < 1e-4
-                assert maxerr(ov["wav"], seq["wav"]) < 1e-3
-    finally:
-        for k, v in saved.items():
-            os.environ.pop(k, None) if v is None else os.environ.__setitem__(k, v)
 
 
 def test_graph_replay_matches_eager(PLM, ADM):

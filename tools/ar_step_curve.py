@@ -70,8 +70,7 @@ def main():
             print(json.dumps({"stack": name, "B": a.batch, "S": S, "rows": a.batch * S, "ms_per_step": round(ms, 3),
                               "gflop": round(fl / 1e9, 1), "tflops_fp32_equiv": round(fl / ms / 1e9, 1),
                               "launches": (ops.launch_count() - n0) // a.reps}), flush=True)
-        row = {"stack": name, "sum_ms_over_listed_steps": round(tot_ms, 2), "steps": len(a.steps),
-               "model": os.environ.get("MEGATTS2_TC_MODEL", "1")}
+        row = {"stack": name, "sum_ms_over_listed_steps": round(tot_ms, 2), "steps": len(a.steps)}
         if a.infer:
             tc = torch.relu(torch.randn(a.batch, 64, 512, generator=g)).to(DEV)
             row["infer_T64_ms"] = timed_infer((plm if name == "plm" else adm).infer, tc)

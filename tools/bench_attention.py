@@ -1,5 +1,5 @@
-"""A/B of the two attention kernels (diagnostics, GPU only): fp32 FFMA kernel (ops.cu) vs tcgen05 kernel (attn_tc.cu)
-at the PLM / ADM head shapes, sequence lengths 32 .. 512.  One process per kernel (the switch is read once)."""
+"""Attention time per shape (diagnostics, GPU only) at the PLM / ADM head shapes, sequence lengths 32 .. 512, through the
+default dispatch: the fp32 kernel (ops.cu) up to 64 queries, the tcgen05 kernel (attn_tc.cu) above."""
 import os
 import sys
 import time
@@ -11,7 +11,6 @@ from megatts2_b200 import ops  # noqa: E402
 
 
 def main():
-    mode = os.environ.get("MEGATTS2_ATTN_TC", "1")
     for (B, H, dh) in ((64, 16, 64), (64, 8, 96), (16, 16, 64)):
         for S in [int(x) for x in os.environ.get("BENCH_S", "32,64,128,256,512").split(",")]:
             if B * S > 64 * 256 and B == 64:
@@ -30,7 +29,7 @@ def main():
             torch.cuda.synchronize()
             ms = e0.elapsed_time(e1) / 20
             fl = 4.0 * B * H * S * S * dh
-            print(f"ATTN_TC={mode} PAIR_MIN={os.environ.get('MEGATTS2_ATTN_PAIR_MIN', '24')} B{B} H{H} dh{dh} S{S:4d}: {ms * 1e3:8.1f} us  {fl / ms / 1e9:7.2f} TFLOP/s", flush=True)
+            print(f"B{B} H{H} dh{dh} S{S:4d}: {ms * 1e3:8.1f} us  {fl / ms / 1e9:7.2f} TFLOP/s", flush=True)
 
 
 if __name__ == "__main__":

@@ -1,6 +1,6 @@
-"""Per-shape throughput of the tensor-core tap-GEMM under the engine's tuning switches (diagnostics, GPU only).
+"""Per-shape throughput of the tensor-core tap-GEMM with the launch plan the dispatcher picks (diagnostics, GPU only).
 
-For each (shape, variant) runs the op `reps` times inside the library's event trace and reports the main kernel's
+For each shape runs the op `reps` times inside the library's event trace and reports the main kernel's
 time per launch (the activation split is traced separately) and its rate in fp32-equivalent TFLOP/s
 (2*M*N*K*k; the tensor pipe executes 6 bf16 MMAs per fp32 product, so dense-bf16-equivalent = 6x).
 """
@@ -33,12 +33,6 @@ SHAPES = [
     dict(name="adm qkv  M4096 K768  N2304", B=1, T=4096, Cin=768, Cout=2304, k=1),
     dict(name="adm ff1  M4096 K768  N1024", B=1, T=4096, Cin=768, Cout=1024, k=1),
 ]
-VARIANTS = [
-    ("single-CTA, 64-wide K-slabs", dict(MEGATTS2_TC_PAIR="0", MEGATTS2_TC_SWB64="0")),
-    ("single-CTA, 32-wide K-slabs", dict(MEGATTS2_TC_PAIR="0", MEGATTS2_TC_SWB64="1")),
-    ("CTA pair,   64-wide K-slabs", dict(MEGATTS2_TC_PAIR="3", MEGATTS2_TC_SWB64="0")),
-    ("CTA pair,   32-wide K-slabs", dict(MEGATTS2_TC_PAIR="4", MEGATTS2_TC_SWB64="0")),
-]
 
 
 def trace_ms(fn, reps):
@@ -64,7 +58,6 @@ def main():
     ap.add_argument("--reps", type=int, default=10)
     ap.add_argument("--shapes", type=str, default="", help="comma-separated shape indices (default: all)")
     ap.add_argument("--fmt", type=str, default="f16x2", choices=["f16x2", "bf16x3"])
-    ap.add_argument("--variants", type=str, default="", help="comma-separated variant indices (default: all)")
     args = ap.parse_args()
     reps = args.reps
     shapes = [SHAPES[int(i)] for i in args.shapes.split(",")] if args.shapes else SHAPES
@@ -80,12 +73,9 @@ def main():
         wp, wt = pack.pack_conv(w.to(DEV)), pack.pack_conv_tc_planes(w.to(DEV), fmt)
         out = torch.empty(s["B"], s["T"], s["Cout"], device=DEV)
         flops = 2.0 * s["B"] * s["T"] * s["Cin"] * s["Cout"] * k
-        variants = [VARIANTS[int(i)] for i in args.variants.split(",")] if args.variants else VARIANTS
-        for vname, env in variants:
-            os.environ.update(env)
-            ms = trace_ms(lambda: ops.conv1d(x, wp, b, out=out, w_tc=wt, k=k, dil=dil, pad=pad, pad_mode=1 if k > 1 else 0), reps)
-            print(f"{s['name']:30s} {vname:30s} {ms:8.3f} ms  {flops / ms / 1e9:7.1f} TFLOP/s fp32-equiv "
-                  f"({nm * flops / ms / 1e9:7.0f} dense 16-bit, {args.fmt})", flush=True)
+        ms = trace_ms(lambda: ops.conv1d(x, wp, b, out=out, w_tc=wt, k=k, dil=dil, pad=pad, pad_mode=1 if k > 1 else 0), reps)
+        print(f"{s['name']:30s} {ms:8.3f} ms  {flops / ms / 1e9:7.1f} TFLOP/s fp32-equiv "
+              f"({nm * flops / ms / 1e9:7.0f} dense 16-bit, {args.fmt})", flush=True)
         del x, out
         torch.cuda.empty_cache()
 
